@@ -3,6 +3,7 @@
 
   python bench.py --gpus N --steps K --warmup W [--config C2|C3|C5]     B200 arm (N>1: launched by torch.distributed.run)
   python bench.py --impl reference --gpus N --steps K ...               the reference's CPU implementation of the path
+  python bench.py ... --dump-outputs DIR                                 also write what the last timed step computed, DIR/<name>.npy
 
 Workloads (BASELINE.json `configs`): C2 (default, configs[1], the one `metric` is quoted on): 4-channel 128^3 volumes,
 UNet3D base_width=32, bf16 tensor-core operands / fp32 accumulate, batch 2 per GPU, one step = forward, sigmoid-Dice,
@@ -26,6 +27,7 @@ import sys
 import tempfile
 import time
 
+import numpy as np
 import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
@@ -53,6 +55,23 @@ CONFIGS = {
 # tools/gpu_trip_prof.sh + tools/summarize_ncu.py when the kernel or the dispatch changes
 NCU_TRAFFIC = {"bytes_per_launch": 339.6e6, "source": "profiles/r02_launches.txt (ncu dram__bytes_read.sum + dram__bytes_write.sum, "
                                                       "mean over the kernel's launches of one C2 step)"}
+
+
+# --dump-outputs keeps at most this many elements of one array (16 MiB in float32), so that a dump stays under 64 MB
+DUMP_SAMPLE = 1 << 22
+
+
+def dump_outputs(path, arrays):
+    """Writes each tensor as float32 ``path/<name>.npy``.  A tensor of more than DUMP_SAMPLE elements is replaced by its
+    flattened elements at DUMP_SAMPLE fixed positions (the first entries of a seed-0 permutation, ascending), the same
+    positions in every run of the same workload, so that two builds can be compared output for output."""
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        t = t.detach()
+        if t.numel() > DUMP_SAMPLE:
+            idx = torch.randperm(t.numel(), generator=torch.Generator().manual_seed(0))[:DUMP_SAMPLE].sort().values
+            t = t.reshape(-1)[idx.to(t.device)]
+        np.save(os.path.join(path, name + ".npy"), t.float().cpu().numpy())
 
 
 def env_rank():
@@ -307,18 +326,19 @@ def run_b200_arm(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """Milliseconds of ``steps`` calls of ``fn`` (max over ranks) and what the last call returned."""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            last = fn()
         e1.record()
         torch.cuda.synchronize()
         ms = torch.tensor([e0.elapsed_time(e1)], device=dev)
         if world > 1:
             dist.all_reduce(ms, op=dist.ReduceOp.MAX)
         barrier()
-        return float(ms.item())
+        return float(ms.item()), last
 
     torch.manual_seed(0)
     model = pkg.UNet3D(precision=args.precision, **cfg["model"]).to(dev)
@@ -367,7 +387,12 @@ def run_b200_arm(args):
             step_resident()
         if rank == 0:
             sampler.start()
-        ms_total = timed(step_resident, args.steps)
+        ms_total, loss = timed(step_resident, args.steps)
+        if args.dump_outputs and rank == 0:
+            # what the step hands its caller: the loss, the gradients (flat, in state-dict order) and the updated parameters
+            params = model.ordered_parameters()
+            dump_outputs(args.dump_outputs, {"loss": loss, "gradients": torch.cat([p.grad.reshape(-1) for p in params]),
+                                             "parameters": torch.cat([p.detach().reshape(-1) for p in params])})
         plan = model._plan_for(x)
         launches_per_step = model.launches_last_forward + model.launches_last_backward + 3   # + Dice sums/finalize/bwd
 
@@ -381,7 +406,7 @@ def run_b200_arm(args):
                                             use_cuda_graph=use_graph)
         pkg.train.epoch_training(loader[:3], model, crit, opt, epoch=0, n_gpus=1, print_frequency=0, grad_sync=sync,
                                  use_cuda_graph=use_graph)
-        ms_e2e = timed(epoch, 1)
+        ms_e2e, _ = timed(epoch, 1)
         clocks = sampler.stop() if rank == 0 else None
         h2d = int(xh.numel() * 4 + th.numel())
         d2h = 4
@@ -409,7 +434,9 @@ def run_b200_arm(args):
             step_resident()
         if rank == 0:
             sampler.start()
-        ms_total = timed(step_resident, args.steps)
+        ms_total, prediction = timed(step_resident, args.steps)
+        if args.dump_outputs and rank == 0:
+            dump_outputs(args.dump_outputs, {"prediction": prediction})
         tiles = torch.empty((cfg["sw_batch"], cfg["model"]["n_features"]) + cfg["roi"], device=dev)
         plan = model._plan_for(tiles, inference_only=True)
         n_fwd = 27 // cfg["sw_batch"]
@@ -426,7 +453,7 @@ def run_b200_arm(args):
         def e2e_step():
             pkg.volumetric_predictions(model, [{"image": xp}], None, activation="sigmoid", inferer=inf, writer=writer)
         e2e_step()
-        ms_e2e = timed(e2e_step, args.steps)
+        ms_e2e, _ = timed(e2e_step, args.steps)
         clocks = sampler.stop() if rank == 0 else None
         h2d = int(xh.numel() * 4)
         d2h = int(host_out.numel() * 4)
@@ -524,6 +551,9 @@ def main():
     ap.add_argument("--precision", default="bf16", choices=["bf16", "split"])
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--no-graph", action="store_true", help="eager launches instead of the CUDA-graph replayed step")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="after the timed steps, write what the last one computed as float32 "
+                    "DIR/<name>.npy (training: loss, gradients, parameters; inference: prediction), at most %d elements each "
+                    "(a fixed sample of a larger array)" % DUMP_SAMPLE)
     args = ap.parse_args()
     if args.impl == "reference":
         run_reference_arm(args)

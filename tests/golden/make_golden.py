@@ -1,6 +1,6 @@
 """Generate the committed golden fixtures by running the UNMODIFIED reference UNet3D on CPU.
 
-Run in the build container (needs /root/reference):   python tests/golden/make_golden.py
+Needs the reference source tree (located by oracle/ref_loader.py):   python tests/golden/make_golden.py
 Writes tests/golden/*.npz .  Inputs/weights are NOT stored: they are regenerated from seeds by
 ``oracle.make_state_dict`` / ``golden_inputs`` so the fixtures stay small.
 """
@@ -18,7 +18,7 @@ from oracle import UNetConfig, make_state_dict, unet3d_state_dict_spec, dice_los
 from oracle.ref_loader import reference_unet3d  # noqa: E402
 
 sys.path.insert(0, HERE)
-from recipe import CASES, golden_inputs, dropout_mask  # noqa: E402
+from recipe import CASES, REFERENCE_CASES, SUB2, golden_inputs, dropout_mask, reference_eval_input  # noqa: E402
 
 
 def run_case(name, kw, shape, dtype):
@@ -76,6 +76,25 @@ def main():
         path = os.path.join(HERE, name + ".npz")
         np.savez_compressed(path, **out)
         print(name, "dice", float(loss), "fp32 rel", rel32, "->", os.path.getsize(path), "bytes")
+    reference_unet3d_fixture()
+
+
+def reference_unet3d_fixture():
+    out = {}
+    for name, (kw, shape) in REFERENCE_CASES.items():
+        model = reference_unet3d(**kw).double()
+        sd = model.state_dict()
+        out["keys::" + name] = np.array(list(sd))
+        out["shapes::" + name] = np.array(["x".join(str(d) for d in v.shape) for v in sd.values()])
+        model.load_state_dict(make_state_dict(UNetConfig(**kw), seed=3, dtype=torch.float64), strict=True)
+        model.eval()
+        with torch.no_grad():
+            y = model(reference_eval_input(shape))
+        out["eval_sub2::" + name] = y[SUB2].numpy()
+        out["eval_norm::" + name] = np.float64(y.norm())
+    path = os.path.join(HERE, "reference_unet3d.npz")
+    np.savez_compressed(path, **out)
+    print("reference_unet3d ->", os.path.getsize(path), "bytes")
 
 
 if __name__ == "__main__":

@@ -11,6 +11,25 @@ CASES = {
 }
 
 
+# reference_unet3d.npz: the reference UNet3D's state-dict spec and eval-mode forward (weights make_state_dict(seed=3), fp64
+# input from seed 5) per case; the forward is stored at every second voxel along each spatial axis, plus its full norm
+REFERENCE_CASES = {
+    "bw8_16": (dict(n_features=4, n_outputs=3, base_width=8), (1, 4, 16, 16, 16)),
+    "bw8_3lev_n2_16x24x16": (dict(n_features=2, n_outputs=2, base_width=8, encoder_blocks=[1, 1, 2]), (2, 2, 16, 24, 16)),
+    "bw8_convT_16": (dict(n_features=4, n_outputs=3, base_width=8, use_transposed_convolutions=True), (1, 4, 16, 16, 16)),
+}
+SUB2 = (slice(None), slice(None), slice(None, None, 2), slice(None, None, 2), slice(None, None, 2))
+
+
+def reference_eval_input(shape):
+    return torch.randn(shape, dtype=torch.float64, generator=torch.Generator().manual_seed(5))
+
+
+def stored_spec(gold, name):
+    """The reference's ordered (key, shape) state-dict spec of case ``name`` from reference_unet3d.npz."""
+    return [(str(k), tuple(int(d) for d in str(s).split("x") if d)) for k, s in zip(gold["keys::" + name], gold["shapes::" + name])]
+
+
 def golden_inputs(shape, n_outputs, seed=1):
     g = torch.Generator().manual_seed(seed)
     x = torch.randn(shape, generator=g, dtype=torch.float32)

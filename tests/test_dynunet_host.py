@@ -1,8 +1,5 @@
 """Host logic of the DynUNet mirror (no GPU): MONAI kwarg surface, state-dict spec == the restated oracle spec == the
 library plan's spec, loud rejection of what is not implemented, the reference's JSON config builds."""
-import json
-import os
-
 import pytest
 import torch
 
@@ -40,13 +37,10 @@ def test_unimplemented_options_raise(pkg, bad):
 
 
 def test_reference_example_config_builds(pkg):
-    path = "/root/reference/examples/brats2020/brats2020_config.json"
-    if os.path.exists(path):
-        cfg = json.load(open(path))["model"]
-    else:   # the GPU box has no /root/reference: the same model block, restated
-        cfg = dict(name="DynUNet", in_channels=4, out_channels=3, spatial_dims=3, deep_supervision=False,
-                   strides=[[1, 1, 1]] + [[2, 2, 2]] * 5, filters=[64, 96, 128, 192, 256, 384], kernel_size=[[3, 3, 3]] * 6,
-                   upsample_kernel_size=[[2, 2, 2]] * 5)
+    # the "model" block of the reference's examples/brats2020/brats2020_config.json
+    cfg = dict(name="DynUNet", in_channels=4, out_channels=3, spatial_dims=3, deep_supervision=False,
+               strides=[[1, 1, 1]] + [[2, 2, 2]] * 5, filters=[64, 96, 128, 192, 256, 384], kernel_size=[[3, 3, 3]] * 6,
+               upsample_kernel_size=[[2, 2, 2]] * 5)
     name = cfg.pop("name")
     m = pkg.fetch_model_by_name(name, **cfg)
     assert m.filters == [64, 96, 128, 192, 256, 384]

@@ -1,13 +1,17 @@
 """Host-side mirror of the reference interface (CPU only): factories, state-dict handling, error behaviour, the
 step loop and the inference contract.  The CUDA path itself is exercised by the -m gpu tests."""
 import os
+import sys
 
+import numpy as np
 import pytest
 import torch
 from torch import nn
 
 from oracle import UNetConfig, make_state_dict, sliding_window_inference
-from oracle.ref_loader import reference_available, reference_unet3d
+
+sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
+from recipe import REFERENCE_CASES, stored_spec  # noqa: E402
 
 
 def test_fetch_model_by_name(pkg):
@@ -54,14 +58,18 @@ def test_state_dict_roundtrip_and_build_or_load(pkg, tmp_path):
     assert torch.equal(w[:, 2:], sd_small["encoder.layers.0.blocks.0.conv1.conv.weight"])
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not mounted (GPU box)")
-def test_checkpoint_interchange_with_reference(pkg):
-    kw = dict(n_features=4, n_outputs=3, base_width=8)
-    ref = reference_unet3d(**kw)
+def test_checkpoint_interchange_with_reference(pkg, golden_dir):
+    """Checkpoints move both ways between the reference UNet3D and this module: the two state dicts have the same keys, in
+    the same order, with the same shapes (the reference's, stored in tests/golden/reference_unet3d.npz)."""
+    kw, _ = REFERENCE_CASES["bw8_16"]
+    spec = stored_spec(np.load(os.path.join(golden_dir, "reference_unet3d.npz")), "bw8_16")
+    g = torch.Generator().manual_seed(0)
+    ref_sd = {k: torch.randn(shape, generator=g) for k, shape in spec}
     mine = pkg.UNet3D(**kw)
-    mine.load_state_dict(ref.state_dict(), strict=True)           # reference checkpoint -> B200 module
-    ref.load_state_dict(mine.state_dict(), strict=True)           # and back
-    assert list(mine.state_dict()) == list(ref.state_dict())
+    mine.load_state_dict(ref_sd, strict=True)                     # reference checkpoint -> B200 module
+    assert [(k, tuple(v.shape)) for k, v in mine.state_dict().items()] == spec      # and back
+    for k, v in mine.state_dict().items():
+        assert torch.equal(v, ref_sd[k]), k
 
 
 def test_default_init_matches_torch_bounds(pkg):

@@ -1,6 +1,6 @@
 """The oracle (CPU restatement) against the committed golden fixtures, which were produced by the UNMODIFIED
-reference UNet3D (tests/golden/make_golden.py).  Also, when /root/reference is present (build container), pins the
-restatement against the live reference class directly."""
+reference UNet3D (tests/golden/make_golden.py): training-mode forward, Dice and gradients, and the reference's state-dict
+spec and eval-mode forward."""
 import os
 import sys
 
@@ -9,10 +9,9 @@ import pytest
 import torch
 
 from oracle import UNetConfig, make_state_dict, unet3d_forward, unet3d_state_dict_spec, dice_loss
-from oracle.ref_loader import reference_available, reference_unet3d
 
 sys.path.insert(0, os.path.join(os.path.dirname(__file__), "golden"))
-from recipe import CASES, golden_inputs, dropout_mask  # noqa: E402
+from recipe import CASES, REFERENCE_CASES, SUB2, golden_inputs, dropout_mask, reference_eval_input, stored_spec  # noqa: E402
 
 FAST = ["c1_bw8_32", "bw16_n2_32", "bw8_convT_32", "c5like_1ch_5lev_32", "bw8_nonpow2_24x32x40"]
 
@@ -69,21 +68,14 @@ def test_state_dict_spec_counts():
     assert abs(sum(int(np.prod(s)) for _, s in spec_t) - 25.35e6) < 0.02e6
 
 
-@pytest.mark.skipif(not reference_available(), reason="reference tree not mounted (GPU box)")
-@pytest.mark.parametrize("kw,shape", [
-    (dict(n_features=4, n_outputs=3, base_width=8), (1, 4, 16, 16, 16)),
-    (dict(n_features=2, n_outputs=2, base_width=8, encoder_blocks=[1, 1, 2]), (2, 2, 16, 24, 16)),
-    (dict(n_features=4, n_outputs=3, base_width=8, use_transposed_convolutions=True), (1, 4, 16, 16, 16)),
-])
-def test_oracle_matches_live_reference(kw, shape):
+@pytest.mark.parametrize("name", sorted(REFERENCE_CASES))
+def test_oracle_matches_reference_fixture(name, golden_dir):
+    gold = np.load(os.path.join(golden_dir, "reference_unet3d.npz"))
+    kw, shape = REFERENCE_CASES[name]
     cfg = UNetConfig(**kw)
-    ref = reference_unet3d(**kw).double()
-    assert [(k, tuple(v.shape)) for k, v in ref.state_dict().items()] == unet3d_state_dict_spec(cfg)
+    assert stored_spec(gold, name) == unet3d_state_dict_spec(cfg)
     sd = make_state_dict(cfg, seed=3, dtype=torch.float64)
-    ref.load_state_dict(sd, strict=True)
-    ref.eval()
-    x = torch.randn(shape, dtype=torch.float64, generator=torch.Generator().manual_seed(5))
     with torch.no_grad():
-        a = ref(x)
-        b = unet3d_forward(sd, x, cfg)
-    assert float((a - b).abs().max()) < 1e-10
+        b = unet3d_forward(sd, reference_eval_input(shape), cfg)
+    assert float(np.abs(b[SUB2].numpy() - gold["eval_sub2::" + name]).max()) < 1e-10
+    assert abs(float(b.norm()) - float(gold["eval_norm::" + name])) <= 1e-12 * float(gold["eval_norm::" + name])
